@@ -40,10 +40,10 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
-    """The unmodified reference objects (oracle/_ref); absent only if nobody ran oracle/refbuild/build_ref.sh where /root/reference exists."""
+    """The unmodified reference objects (oracle/_ref); built by build() where the 3DWorld sources exist (REFERENCE_ROOT, else BASELINE.json's reference_path)."""
     import refapi as R
     if not R.available():
-        pytest.skip("oracle/_ref/libref3dworld.so not built")
+        pytest.skip("oracle/_ref/libref3dworld.so not built (build() builds it where the 3DWorld sources exist: REFERENCE_ROOT, else BASELINE.json's reference_path)")
     R.lib().ref_set_threads(max(1, min(16, os.cpu_count() or 1)))
     return R
 

@@ -1,10 +1,19 @@
 """GPU parity: tw_heightgen_2d / tw_heightgen_tiles (CUDA, through the C ABI) vs the CPU oracle - bit-exact for every gen mode."""
+import importlib.util
+import json
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 
 from cases import convert, height_cases, HM_CFG
+from test_oracle_golden import hp_from_args
 
 pytestmark = pytest.mark.gpu
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLD = os.path.join(ROOT, "tests", "golden")
 
 
 def _run_case(tw, scene, oracle, ctx, kw, org, size, sp_cache={}):
@@ -113,8 +122,54 @@ def test_full_size_properties(tw, scene, oracle, ctx, beq):
     assert beq(out[6000:6064, 4000:4096].cpu().numpy(), zc) == 0
 
 
-def test_matches_linked_reference(tw, scene, ref, ctx, beq):
-    """Directly against the unmodified reference objects (oracle/_ref travels to the GPU box as a prebuilt .so)."""
+def _bench_kernel_only(steps, dump_dir):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1", "--kernel-only",
+                        "--dump-outputs", str(dump_dir)], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-2000:]
+    return json.loads(r.stdout.strip().splitlines()[-1])
+
+
+def test_bench_dump_outputs(tw, scene, oracle, ctx, beq, tmp_path):
+    """bench.py --dump-outputs writes the headline grid's rows (== the oracle, bit for bit) and its min/max, float32, within 64 MB; --steps sets the
+    number of timed steps (the launches in the timed region scale with it) and does not change what is written."""
+    d2, d3 = tmp_path / "steps2", tmp_path / "steps3"
+    r2, r3 = _bench_kernel_only(2, d2), _bench_kernel_only(3, d3)
+    assert r2["gpu_launches"] > 0 and 3 * r2["gpu_launches"] == 2 * r3["gpu_launches"], (r2["gpu_launches"], r3["gpu_launches"])
+    assert sorted(os.listdir(d2)) == sorted(os.listdir(d3)) == ["height_rows.npy", "minmax.npy"]
+    for name in os.listdir(d2):
+        assert np.load(d2 / name).tobytes() == np.load(d3 / name).tobytes(), name
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rows, mm = np.load(d2 / "height_rows.npy"), np.load(d2 / "minmax.npy")
+    assert sum(f.stat().st_size for f in d2.iterdir()) <= 64 << 20
+    assert rows.dtype == mm.dtype == np.float32 and rows.shape == (bench.DUMP_ROWS, bench.N_TILE) and mm.shape == (2,)
+    assert mm[0] <= rows.min() and rows.max() <= mm[1]
+    cfg = scene.SceneConfig(mesh_gen_mode=4, mesh_freq_filter=1, mesh_seed=1, hmap=HM_CFG, zmax_est=2.3)
+    hp = convert(cfg.height_params(), oracle.HeightParams)
+    g = cfg.heightmap_grid(bench.N_TILE, bench.N_TILE)
+    idx = bench.dump_rows()
+    for i in (0, len(idx) // 2, len(idx) - 1):
+        zc = oracle.heightgen_2d(oracle.Grid2D(g.x0, g.y0 + int(idx[i]), g.dx, g.dy, bench.N_TILE, 1), hp, None, 1, 0)
+        assert beq(rows[i], zc) == 0, int(idx[i])
+
+
+def test_matches_linked_reference(tw, scene, ctx, beq, request):
+    """Directly against the unmodified reference: its linked objects (oracle/_ref) when they are built, otherwise the height grids it produced for
+    tests/golden/height.npz (every gen mode and shape, tests/golden/make_golden.py)."""
+    import refapi
+    if not refapi.available():
+        h = np.load(os.path.join(GOLD, "height.npz"))
+        for mode in range(5):
+            for shape in range(3):
+                n = "h_m%d_s%d" % (mode, shape)
+                a = h[n + "_args"]
+                if mode == 0:
+                    ctx.set_sine_params(h[n + "_sp"])
+                g = tw.Grid2D(float(a[4]), float(a[5]), 0.0625, 0.0625, int(a[6]), int(a[7]))
+                assert beq(ctx.heightgen_2d(g, hp_from_args(tw, a, h[n + "_hmap"])), h[n]) == 0, n
+        return
+    ref = request.getfixturevalue("ref")
     for mode in (0, 1, 2, 4):
         ref.setup(mode=mode, freq_filter=1, seed=1, zmax_est=2.3, hmap=HM_CFG)
         cfg = scene.SceneConfig(mesh_gen_mode=mode, mesh_freq_filter=1, mesh_seed=1, hmap=HM_CFG, zmax_est=2.3)
