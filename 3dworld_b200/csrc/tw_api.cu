@@ -44,6 +44,42 @@ bool tw_is_device_ptr(const void *p) {
 	return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged);
 }
 
+bool tw_stage::add(void *d, const void *caller, size_t bytes, size_t slack, int dir) {
+	bool const host = (dir & TEMP) || is_host(caller);
+	if (n_ < MAX_BUFFERS) {e_[n_] = entry{d, caller, nullptr, bytes, host ? tw_align256(bytes + slack) : 0, host ? dir : 0, host};}
+	++n_; // commit() rejects more than MAX_BUFFERS
+	return host;
+}
+
+int tw_stage::commit() {
+	if (n_ > MAX_BUFFERS) return tw_set_error(ctx_, TW_ERR_STATE, "tw_stage: more than %d buffers", (int)MAX_BUFFERS);
+	size_t total = 0;
+	for (int i = 0; i < n_; ++i) {total += e_[i].region;}
+	if (total) {
+		if (ctx_->scratch0_held) return tw_set_error(ctx_, TW_ERR_STATE, "scratch slot 0 holds the buffers of the calling entry point: a nested call must pass device pointers");
+		int const rc = tw_reserve(ctx_, 0, total); if (rc) return rc;
+		held_ = ctx_->scratch0_held = true;
+	}
+	char *q = (char *)ctx_->d_scratch[0];
+	for (int i = 0; i < n_; ++i) {
+		entry &e = e_[i];
+		e.dev = e.host ? (void *)q : const_cast<void *>(e.caller);
+		memcpy(e.d, &e.dev, sizeof(void *)); // e.d is the call site's T* variable
+		q += e.region;
+		if (e.dir & IN) {TW_CUDA(ctx_, cudaMemcpyAsync(e.dev, e.caller, e.bytes, cudaMemcpyHostToDevice, ctx_->stream));}
+	}
+	return TW_OK;
+}
+
+int tw_stage::finish() {
+	for (int i = 0; i < n_; ++i) {
+		entry const &e = e_[i];
+		if (e.dir & OUT) {TW_CUDA(ctx_, cudaMemcpyAsync(const_cast<void *>(e.caller), e.dev, e.bytes, cudaMemcpyDeviceToHost, ctx_->stream));}
+	}
+	TW_CUDA(ctx_, cudaStreamSynchronize(ctx_->stream));
+	return TW_OK;
+}
+
 int twi_ensure_aux_streams(tw_ctx *ctx) {
 	if (ctx->aux_stream[0]) return TW_OK;
 	int lo = 0, hi = 0; // the latency-bound droplet kernels / band copies get the higher priority
@@ -65,9 +101,20 @@ int check_ctx(tw_ctx *ctx) { // NOTE: makes ctx->device the calling thread's cur
 	return TW_OK;
 }
 
-int finish_pending(tw_ctx *ctx) { // complete an outstanding tw_heightgen_2d_launch before other work reuses the scratch buffers
-	if (ctx->async.pending) {return tw_heightgen_2d_poll(ctx, 1);}
-	return TW_OK;
+int single_minmax(tw_ctx *ctx, unsigned **d_mm) { // the one (min, max) pair of slot 2, initialised for a reduction
+	int const rc = tw_reserve(ctx, 2, OFF_TILES); if (rc) return rc;
+	*d_mm = (unsigned *)((char *)ctx->d_scratch[2] + OFF_MM);
+	return twi_init_minmax(ctx, *d_mm, 1);
+}
+
+// setup_height_gen_async / build_arrays((x1 - MESH_X_SIZE/2), (y1 - MESH_Y_SIZE/2), dx, dy, ...): int -> float, then mx0 = dx*x0 (src/tiled_mesh.cpp:461, src/mesh_gen.cpp:591)
+std::vector<float2> tile_origins(const int32_t *origins_xy, uint32_t ntiles, int mesh_x_size, int mesh_y_size, float dx, float dy) {
+	std::vector<float2> org(ntiles);
+	for (uint32_t t = 0; t < ntiles; ++t) {
+		float const x0 = (float)(origins_xy[2*t] - mesh_x_size/2), y0 = (float)(origins_xy[2*t+1] - mesh_y_size/2);
+		org[t] = make_float2(dx*x0, dy*y0);
+	}
+	return org;
 }
 
 int read_minmax(tw_ctx *ctx, const unsigned *d_mm, tw_minmax *mm, uint32_t n) { // synchronous
@@ -90,6 +137,12 @@ int validate_height(tw_ctx *ctx, const tw_grid2d *g, const tw_height_params *p, 
 }
 
 } // namespace
+
+int tw_enter(tw_ctx *ctx) {
+	int const rc = check_ctx(ctx); if (rc) return rc;
+	if (ctx->async.pending) {return tw_heightgen_2d_poll(ctx, 1);} // an outstanding tw_heightgen_2d_launch completes before other work reuses the scratch buffers
+	return TW_OK;
+}
 
 extern "C" {
 
@@ -176,18 +229,16 @@ int tw_set_sine_params(tw_ctx *ctx, const float *sp) {
 
 // ------------------------------------------------------------------------------------------------ 2-D height
 int tw_heightgen_2d_launch(tw_ctx *ctx, const tw_grid2d *g, const tw_height_params *p, int enable_glaciate, int min_start_sin, float *out, tw_minmax *mm) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	rc = validate_height(ctx, g, p, out); if (rc) return rc;
-	size_t const n = (size_t)g->nx*g->ny;
-	bool const dev_out = tw_is_device_ptr(out);
-	float *d_out = out;
-	if (!dev_out) {rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc; d_out = (float *)ctx->d_scratch[0];}
-	rc = tw_reserve(ctx, 2, OFF_TILES); if (rc) return rc;
-	unsigned *d_mm = mm ? (unsigned *)((char *)ctx->d_scratch[2] + OFF_MM) : nullptr;
-	if (d_mm) {rc = twi_init_minmax(ctx, d_mm, 1); if (rc) return rc;}
-	if (!dev_out) {rc = twi_ensure_aux_streams(ctx); if (rc) return rc;}
-	rc = twi_heightgen(ctx, g, p, enable_glaciate, min_start_sin, nullptr, 1, d_out, d_mm, dev_out ? nullptr : out); // host out: band-wise D2H overlapped with compute
+	float *d_out;
+	tw_stage st(ctx);
+	bool const host_out = st.view(&d_out, out, (size_t)g->nx*g->ny*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	unsigned *d_mm = nullptr;
+	if (mm) {rc = single_minmax(ctx, &d_mm); if (rc) return rc;}
+	if (host_out) {rc = twi_ensure_aux_streams(ctx); if (rc) return rc;}
+	rc = twi_heightgen(ctx, g, p, enable_glaciate, min_start_sin, nullptr, 1, d_out, d_mm, host_out ? out : nullptr); // host out: band-wise D2H overlapped with compute
 	if (rc) return rc;
 	if (mm) {
 		rc = tw_reserve_pinned(ctx, 2*sizeof(unsigned)); if (rc) return rc;
@@ -229,8 +280,7 @@ int tw_heightgen_2d(tw_ctx *ctx, const tw_grid2d *g, const tw_height_params *p, 
 int tw_tile_weights_batch(tw_ctx *ctx, const float *zvals, const int32_t *origins_xy, uint32_t ntiles, int mesh_x_size, int mesh_y_size, float dx, float dy,
                           uint32_t zvsize, const tw_height_params *p, const tw_weight_params *wp, const float *tile_params, uint8_t *weights, uint8_t *has_any_grass)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!zvals || !origins_xy || !p || !wp || !tile_params || !weights || ntiles == 0 || zvsize < 3) return tw_set_error(ctx, TW_ERR_ARG, "tw_tile_weights_batch: null argument, no tiles or zvsize < 3");
 	tw_weight_params W = *wp;
 	int seen[5] = {0, 0, 0, 0, 0};
@@ -241,64 +291,47 @@ int tw_tile_weights_batch(tw_ctx *ctx, const float *zvals, const int32_t *origin
 	if (!(W.zmax > W.zmin)) return tw_set_error(ctx, TW_ERR_ARG, "zmax must exceed zmin");
 	uint32_t const stride = zvsize - 1;
 	size_t const zn = (size_t)ntiles*zvsize*zvsize, tn = (size_t)ntiles*stride*stride;
-	bool const dev_z = tw_is_device_ptr(zvals), dev_w = tw_is_device_ptr(weights), dev_f = has_any_grass && tw_is_device_ptr(has_any_grass), dev_p = tw_is_device_ptr(tile_params);
-	auto al = [](size_t b) {return (b + 255) & ~(size_t)255;};
-	rc = tw_reserve(ctx, 0, al(tn*sizeof(float)) + (dev_z ? 0 : al(zn*sizeof(float))) + (dev_w ? 0 : al(tn*4)) + al(ntiles) + (dev_p ? 0 : al((size_t)ntiles*8*sizeof(float))) + 256);
-	if (rc) return rc;
-	char *q = (char *)ctx->d_scratch[0];
-	float *d_rand = (float *)q; q += al(tn*sizeof(float));
-	const float *d_z = zvals;
-	if (!dev_z) {TW_CUDA(ctx, cudaMemcpyAsync(q, zvals, zn*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_z = (const float *)q; q += al(zn*sizeof(float));}
-	uint8_t *d_w = weights;
-	if (!dev_w) {d_w = (uint8_t *)q; q += al(tn*4);}
-	uint8_t *d_f = dev_f ? has_any_grass : (uint8_t *)q; q += al(ntiles);
-	const float *d_p = tile_params;
-	if (!dev_p) {TW_CUDA(ctx, cudaMemcpyAsync(q, tile_params, (size_t)ntiles*8*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_p = (const float *)q;}
-	if (has_any_grass) {TW_CUDA(ctx, cudaMemsetAsync(d_f, 0, ntiles, ctx->stream));}
+	float *d_rand; const float *d_z, *d_p; uint8_t *d_w, *d_f;
+	tw_stage st(ctx);
+	st.temp(&d_rand, tn*sizeof(float));
+	st.in(&d_z, zvals, zn*sizeof(float));
+	st.out(&d_w, weights, tn*4);
+	st.out(&d_f, has_any_grass, ntiles);
+	st.in(&d_p, tile_params, (size_t)ntiles*8*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	if (d_f) {TW_CUDA(ctx, cudaMemsetAsync(d_f, 0, ntiles, ctx->stream));}
 	// height_gen.build_arrays((x1 - MESH_X_SIZE/2), (y1 - MESH_Y_SIZE/2), MESH_NOISE_FREQ*DX_VAL, MESH_NOISE_FREQ*DY_VAL, tsize, tsize, 0, 1) (src/tiled_mesh.cpp:1103)
 	float const MESH_NOISE_FREQ = 80.0f;
 	tw_grid2d g; g.x0 = 0; g.y0 = 0; g.dx = MESH_NOISE_FREQ*dx; g.dy = MESH_NOISE_FREQ*dy; g.nx = stride; g.ny = stride;
-	std::vector<float2> org(ntiles);
-	for (uint32_t t = 0; t < ntiles; ++t) {
-		float const x0 = (float)(origins_xy[2*t] - mesh_x_size/2), y0 = (float)(origins_xy[2*t+1] - mesh_y_size/2);
-		org[t] = make_float2(g.dx*x0, g.dy*y0);
-	}
+	std::vector<float2> const org = tile_origins(origins_xy, ntiles, mesh_x_size, mesh_y_size, g.dx, g.dy);
 	tw_height_params ps = *p;
 	ps.gen_mode = TW_MGEN_SINE; ps.gen_shape = 0; // force_sine_mode: gen_mode = MGEN_SINE, gen_shape = 0 (src/mesh_gen.cpp:592-593)
 	rc = twi_heightgen_sine_tiles(ctx, &g, &ps, 0, 50, org.data(), ntiles, d_rand, nullptr);
 	if (rc) return rc;
-	rc = twi_tile_weights(ctx, d_z, d_rand, ntiles, zvsize, d_p, &W, d_w, has_any_grass ? d_f : nullptr);
+	rc = twi_tile_weights(ctx, d_z, d_rand, ntiles, zvsize, d_p, &W, d_w, d_f);
 	if (rc) return rc;
-	if (!dev_w) {TW_CUDA(ctx, cudaMemcpyAsync(weights, d_w, tn*4, cudaMemcpyDeviceToHost, ctx->stream));}
-	if (has_any_grass && !dev_f) {TW_CUDA(ctx, cudaMemcpyAsync(has_any_grass, d_f, ntiles, cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	return st.finish();
 }
 
 int tw_heightgen_tiles(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntiles, int mesh_x_size, int mesh_y_size, float dx, float dy,
                        uint32_t zvsize, const tw_height_params *p, float *out, tw_minmax *mm)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!origins_xy || ntiles == 0) return tw_set_error(ctx, TW_ERR_ARG, "no tiles");
 	tw_grid2d g; g.x0 = 0; g.y0 = 0; g.dx = dx; g.dy = dy; g.nx = zvsize; g.ny = zvsize;
 	rc = validate_height(ctx, &g, p, out); if (rc) return rc;
-	size_t const tile_elems = (size_t)zvsize*zvsize, n = tile_elems*ntiles;
-	bool const dev_out = tw_is_device_ptr(out);
-	float *d_out = out;
-	if (!dev_out) {rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc; d_out = (float *)ctx->d_scratch[0];}
+	size_t const tile_elems = (size_t)zvsize*zvsize;
+	float *d_out;
+	tw_stage st(ctx);
+	st.out(&d_out, out, tile_elems*ntiles*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
 	size_t const mm_bytes = (size_t)ntiles*2*sizeof(unsigned), org_bytes = (size_t)ntiles*sizeof(float2);
 	rc = tw_reserve(ctx, 2, OFF_TILES + mm_bytes + org_bytes); if (rc) return rc;
 	unsigned *d_mm = mm ? (unsigned *)((char *)ctx->d_scratch[2] + OFF_TILES) : nullptr;
 	float2 *d_org = (float2 *)((char *)ctx->d_scratch[2] + OFF_TILES + mm_bytes);
 	if (d_mm) {rc = twi_init_minmax(ctx, d_mm, ntiles); if (rc) return rc;}
-	// setup_height_gen_async: build_arrays((x0 - MESH_X_SIZE/2), (y0 - MESH_Y_SIZE/2), dx, dy, ...): int -> float, then mx0 = dx*x0 (src/tiled_mesh.cpp:461, src/mesh_gen.cpp:591)
+	std::vector<float2> const org = tile_origins(origins_xy, ntiles, mesh_x_size, mesh_y_size, dx, dy);
 	if (p->gen_mode != TW_MGEN_SINE) {
-		std::vector<float2> org(ntiles);
-		for (uint32_t t = 0; t < ntiles; ++t) {
-			float const x0 = (float)(origins_xy[2*t] - mesh_x_size/2), y0 = (float)(origins_xy[2*t+1] - mesh_y_size/2);
-			org[t] = make_float2(dx*x0, dy*y0);
-		}
 		TW_CUDA(ctx, cudaMemcpyAsync(d_org, org.data(), org_bytes, cudaMemcpyHostToDevice, ctx->stream));
 		TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // org is a local vector
 		uint32_t const zmax = 65535;
@@ -309,39 +342,29 @@ int tw_heightgen_tiles(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntiles, 
 		}
 	}
 	else { // sine tables depend on the tile origin only through its column / row: W + H tables for a W x H block of tiles, one grid launch for the batch
-		std::vector<float2> org(ntiles);
-		for (uint32_t t = 0; t < ntiles; ++t) {
-			float const x0 = (float)(origins_xy[2*t] - mesh_x_size/2), y0 = (float)(origins_xy[2*t+1] - mesh_y_size/2);
-			org[t] = make_float2(dx*x0, dy*y0);
-		}
 		rc = twi_heightgen_sine_tiles(ctx, &g, p, 1, 0, org.data(), ntiles, d_out, d_mm);
 		if (rc) return rc;
 	}
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(out, d_out, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
 	if (mm) {rc = read_minmax(ctx, d_mm, mm, ntiles); if (rc) return rc;}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	return st.finish();
 }
 
 // ------------------------------------------------------------------------------------------------ callers' tails
 int tw_tile_bounds_batch(tw_ctx *ctx, const float *zvals, uint32_t ntiles, uint32_t zvsize, float wpz_max, float dx_val, float dy_val, uint32_t size, tw_tile_bounds *out) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!zvals || !out || ntiles == 0 || zvsize < 4) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	if (4*(zvsize/4) >= zvsize) return tw_set_error(ctx, TW_ERR_ARG, "zvsize %u: the last sub-block would end at cell %u (the reference asserts x_end < zvsize, src/tiled_mesh.cpp:520)", zvsize, 4*(zvsize/4));
 	if (ntiles > 65535) return tw_set_error(ctx, TW_ERR_ARG, "at most 65535 tiles per call");
-	size_t const n = (size_t)ntiles*zvsize*zvsize;
 	struct Sub {float zmin, zmax; int wx1, wy1, wx2, wy2;};
-	size_t const sub_bytes = (size_t)ntiles*16*sizeof(Sub);
-	const float *d_z = zvals;
-	bool const dev = tw_is_device_ptr(zvals);
-	rc = tw_reserve(ctx, 0, (dev ? 0 : n*sizeof(float)) + sub_bytes + 256); if (rc) return rc;
-	char *s0 = (char *)ctx->d_scratch[0];
-	if (!dev) {TW_CUDA(ctx, cudaMemcpyAsync(s0, zvals, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_z = (const float *)s0; s0 += (n*sizeof(float) + 255) & ~(size_t)255;}
-	rc = twi_tile_bounds(ctx, d_z, ntiles, zvsize, wpz_max, s0); if (rc) return rc;
 	std::vector<Sub> sub((size_t)ntiles*16);
-	TW_CUDA(ctx, cudaMemcpyAsync(sub.data(), s0, sub_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	const float *d_z; Sub *d_sub;
+	tw_stage st(ctx);
+	st.in(&d_z, zvals, (size_t)ntiles*zvsize*zvsize*sizeof(float));
+	st.temp(&d_sub, sub.size()*sizeof(Sub));
+	rc = st.commit(); if (rc) return rc;
+	rc = twi_tile_bounds(ctx, d_z, ntiles, zvsize, wpz_max, d_sub); if (rc) return rc;
+	TW_CUDA(ctx, cudaMemcpyAsync(sub.data(), d_sub, sub.size()*sizeof(Sub), cudaMemcpyDeviceToHost, ctx->stream));
+	rc = st.finish(); if (rc) return rc;
 	for (uint32_t t = 0; t < ntiles; ++t) { // combine the 16 sub-blocks exactly as the reference's loop does (src/tiled_mesh.cpp:517-540)
 		tw_tile_bounds &b = out[t];
 		b.mzmin = 100.0f; b.mzmax = -100.0f; b.mesh_dz = 0.0f; // FAR_DISTANCE
@@ -363,45 +386,32 @@ int tw_tile_bounds_batch(tw_ctx *ctx, const float *zvals, uint32_t ntiles, uint3
 }
 
 int tw_glaciate_mesh(tw_ctx *ctx, float *mesh, int nx, int ny, int xoff2, int yoff2, int mesh_x_size, int mesh_y_size, const tw_height_params *p, tw_minmax *zbottom_ztop) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!mesh || !p || nx <= 0 || ny <= 0 || ny > 65535) return tw_set_error(ctx, TW_ERR_ARG, "bad argument");
 	if (!ctx->have_sin) return tw_set_error(ctx, TW_ERR_STATE, "tw_set_sin_table() has not been called");
-	size_t const n = (size_t)nx*ny;
-	bool const dev = tw_is_device_ptr(mesh);
-	float *d_mesh = mesh;
-	if (!dev) {
-		rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc;
-		d_mesh = (float *)ctx->d_scratch[0];
-		TW_CUDA(ctx, cudaMemcpyAsync(d_mesh, mesh, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-	}
-	rc = tw_reserve(ctx, 2, OFF_TILES); if (rc) return rc;
-	unsigned *d_mm = (unsigned *)((char *)ctx->d_scratch[2] + OFF_MM);
-	rc = twi_init_minmax(ctx, d_mm, 1); if (rc) return rc;
+	float *d_mesh;
+	tw_stage st(ctx);
+	st.inout(&d_mesh, mesh, (size_t)nx*ny*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	unsigned *d_mm;
+	rc = single_minmax(ctx, &d_mm); if (rc) return rc;
 	rc = twi_glaciate_mesh(ctx, d_mesh, nx, ny, xoff2, yoff2, mesh_x_size, mesh_y_size, p, d_mm); if (rc) return rc;
-	if (!dev) {TW_CUDA(ctx, cudaMemcpyAsync(mesh, d_mesh, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
-	if (zbottom_ztop) {return read_minmax(ctx, d_mm, zbottom_ztop, 1);}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	if (zbottom_ztop) {rc = read_minmax(ctx, d_mm, zbottom_ztop, 1); if (rc) return rc;}
+	return st.finish();
 }
 
 // ------------------------------------------------------------------------------------------------ erosion
 int tw_erode_tiles(tw_ctx *ctx, float *maps, uint32_t ntiles, int xsize, int ysize, const float *min_zvals, float min_zval_all,
                    uint32_t num_iters, const tw_erosion_params *p)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!maps || !p) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
 	if (xsize <= 0 || ysize <= 0 || ntiles == 0) return tw_set_error(ctx, TW_ERR_ARG, "empty heightmap");
 	if (num_iters == 0 || p->erode_amount <= 0.0) {ctx->last_erosion_steps = 0; return TW_OK;} // src/erosion.cpp:16
-	size_t const n = (size_t)xsize*ysize*ntiles;
-	bool const dev = tw_is_device_ptr(maps);
-	float *d_maps = maps;
-	if (!dev) {
-		rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc;
-		d_maps = (float *)ctx->d_scratch[0];
-		TW_CUDA(ctx, cudaMemcpyAsync(d_maps, maps, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-	}
+	float *d_maps;
+	tw_stage st(ctx);
+	st.inout(&d_maps, maps, (size_t)xsize*ysize*ntiles*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
 	float *d_minz = nullptr;
 	if (min_zvals) {
 		rc = tw_reserve(ctx, 2, OFF_TILES + (size_t)ntiles*sizeof(float)); if (rc) return rc;
@@ -411,17 +421,14 @@ int tw_erode_tiles(tw_ctx *ctx, float *maps, uint32_t ntiles, int xsize, int ysi
 	}
 	rc = twi_erode(ctx, d_maps, ntiles, xsize, ysize, d_minz, min_zval_all, num_iters, p);
 	if (rc) return rc;
-	if (!dev) {TW_CUDA(ctx, cudaMemcpyAsync(maps, d_maps, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	return st.finish();
 }
 
 int tw_create_zvals_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntiles, int mesh_x_size, int mesh_y_size, float dx, float dy,
                           uint32_t zvsize, const tw_height_params *p, uint32_t erosion_iters, const tw_erosion_params *ep, float min_zval,
                           float *out, tw_minmax *mm)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!origins_xy || ntiles == 0 || !p || !out) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	bool const erode = (erosion_iters > 0 && ep && ep->erode_amount > 0.0);
 	ctx->last_erosion_steps = 0;
@@ -429,19 +436,19 @@ int tw_create_zvals_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntile
 	tw_grid2d g; g.x0 = 0; g.y0 = 0; g.dx = dx; g.dy = dy; g.nx = zvsize; g.ny = zvsize;
 	rc = validate_height(ctx, &g, p, out); if (rc) return rc;
 	size_t const tile_elems = (size_t)zvsize*zvsize, n = tile_elems*ntiles;
-	bool const dev_out = tw_is_device_ptr(out);
+	float *d_out;
+	tw_stage st(ctx);
 	if (p->gen_mode == TW_MGEN_SINE) { // sine tables live in the same scratch slot as the padded maps: no overlap, plain sequence
-		float *d_out = out;
-		if (!dev_out) {rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc; d_out = (float *)ctx->d_scratch[0];}
+		st.out(&d_out, out, n*sizeof(float));
+		rc = st.commit(); if (rc) return rc;
 		rc = tw_heightgen_tiles(ctx, origins_xy, ntiles, mesh_x_size, mesh_y_size, dx, dy, zvsize, p, d_out, nullptr); if (rc) return rc;
 		rc = tw_erode_tiles(ctx, d_out, ntiles, (int)zvsize, (int)zvsize, nullptr, min_zval, erosion_iters, ep); if (rc) return rc;
 		if (mm) {for (uint32_t t = 0; t < ntiles; ++t) {rc = tw_minmax_f32(ctx, d_out + (size_t)t*tile_elems, tile_elems, mm + t); if (rc) return rc;}}
-		if (!dev_out) {TW_CUDA(ctx, cudaMemcpy(out, d_out, n*sizeof(float), cudaMemcpyDeviceToHost));}
-		return TW_OK;
+		return st.finish();
 	}
 	rc = twi_ensure_aux_streams(ctx); if (rc) return rc;
-	float *d_out = out;
-	if (!dev_out) {rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc; d_out = (float *)ctx->d_scratch[0];}
+	bool const host_out = st.view(&d_out, out, n*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
 	// The pipeline. Work per tile is heavy-tailed (ocean tiles: 1000 droplets x 1 move; mountain tiles: 1e5 moves in one serial chain), and a chain
 	// cannot be sped up (csrc/tw_erosion.cu, plan_heavy), so the chains must START EARLY: (1) a coarse pre-pass evaluates the height function on an
 	// 8x8 sample of every tile (4 M evaluations for 65536 tiles, < 1 ms) and counts the samples above the ocean-stop level - the same predictor the
@@ -465,12 +472,12 @@ int tw_create_zvals_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntile
 	chunk = (ntiles + nchunks - 1)/nchunks; // balanced
 	bool const reorder = (nchunks > 1 && !getenv("TW_PIPE_NO_REORDER"));
 	int const nes = (nchunks > 2) ? 3 : (int)nchunks; // erosion streams / scratch buffers
-	size_t const sbytes = (twi_erode_scratch_bytes(chunk, (int)zvsize, (int)zvsize) + 255) & ~(size_t)255;
+	size_t const sbytes = tw_align256(twi_erode_scratch_bytes(chunk, (int)zvsize, (int)zvsize));
 	rc = tw_reserve(ctx, 1, sbytes*nes); if (rc) return rc;
 	// slot 2: [small scalars | per-tile min/max | origins | sorted origins | work | order | hist(256) | coarse samples]
 	uint32_t const CS = 8, cstep = (zvsize >= CS) ? zvsize/CS : 1;
-	size_t const mm_bytes = ((size_t)ntiles*2*sizeof(unsigned) + 255) & ~(size_t)255, org_bytes = ((size_t)ntiles*sizeof(float2) + 255) & ~(size_t)255;
-	size_t const u_bytes = ((size_t)ntiles*sizeof(unsigned) + 255) & ~(size_t)255, coarse_bytes = reorder ? (((size_t)ntiles*CS*CS*sizeof(float) + 255) & ~(size_t)255) : 0;
+	size_t const mm_bytes = tw_align256((size_t)ntiles*2*sizeof(unsigned)), org_bytes = tw_align256((size_t)ntiles*sizeof(float2));
+	size_t const u_bytes = tw_align256((size_t)ntiles*sizeof(unsigned)), coarse_bytes = reorder ? tw_align256((size_t)ntiles*CS*CS*sizeof(float)) : 0;
 	rc = tw_reserve(ctx, 2, OFF_TILES + mm_bytes + 2*org_bytes + 2*u_bytes + 1024 + coarse_bytes); if (rc) return rc;
 	char *s2 = (char *)ctx->d_scratch[2] + OFF_TILES;
 	unsigned *d_mm = (unsigned *)s2; s2 += mm_bytes;
@@ -482,11 +489,7 @@ int tw_create_zvals_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntile
 	float *d_coarse = (float *)s2;
 	unsigned long long *d_steps = (unsigned long long *)((char *)ctx->d_scratch[2] + 2048);
 	{
-		std::vector<float2> org(ntiles);
-		for (uint32_t t = 0; t < ntiles; ++t) { // build_arrays((x1 - MESH_X_SIZE/2), (y1 - MESH_Y_SIZE/2), ...): int -> float, mx0 = dx*x0 (src/tiled_mesh.cpp:461, src/mesh_gen.cpp:591)
-			float const x0 = (float)(origins_xy[2*t] - mesh_x_size/2), y0 = (float)(origins_xy[2*t+1] - mesh_y_size/2);
-			org[t] = make_float2(dx*x0, dy*y0);
-		}
+		std::vector<float2> const org = tile_origins(origins_xy, ntiles, mesh_x_size, mesh_y_size, dx, dy);
 		TW_CUDA(ctx, cudaMemcpyAsync(d_org, org.data(), (size_t)ntiles*sizeof(float2), cudaMemcpyHostToDevice, ctx->stream));
 		TW_CUDA(ctx, cudaMemsetAsync(d_steps, 0, sizeof(unsigned long long), ctx->stream));
 		TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // org is a local vector; the aux streams must also see d_steps zeroed
@@ -523,13 +526,13 @@ int tw_create_zvals_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntile
 		status = twi_erode_enqueue(ctx, es, 1 + lane, (char *)ctx->d_scratch[1] + (size_t)lane*sbytes, chunk, maps, nt, (int)zvsize, (int)zvsize, nullptr, min_zval, erosion_iters, ep, d_steps, perm_k);
 		if (status) break;
 		if (mm) {status = twi_minmax_tiles(ctx, es, maps, tile_elems, nt, d_perm ? d_mm : d_mm + 2*(size_t)t0, perm_k); if (status) break;}
-		if (!dev_out && !d_perm && cudaMemcpyAsync(out + (size_t)t0*tile_elems, maps, (size_t)nt*tile_elems*sizeof(float), cudaMemcpyDeviceToHost, es) != cudaSuccess) {status = tw_set_error(ctx, TW_ERR_CUDA, "D2H");}
+		if (host_out && !d_perm && cudaMemcpyAsync(out + (size_t)t0*tile_elems, maps, (size_t)nt*tile_elems*sizeof(float), cudaMemcpyDeviceToHost, es) != cudaSuccess) {status = tw_set_error(ctx, TW_ERR_CUDA, "D2H");}
 	}
 	cudaError_t e0 = cudaStreamSynchronize(ctx->stream), e1 = cudaStreamSynchronize(ctx->aux_stream[0]), e2 = cudaStreamSynchronize(ctx->aux_stream[1]), e3 = cudaStreamSynchronize(ctx->aux_stream[2]);
 	for (cudaEvent_t e : ev) {if (e) cudaEventDestroy(e);}
 	if (status) return status;
 	if (e0 != cudaSuccess || e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess) return tw_set_error(ctx, TW_ERR_CUDA, "tile pipeline: %s", cudaGetErrorString(e0 != cudaSuccess ? e0 : (e1 != cudaSuccess ? e1 : (e2 != cudaSuccess ? e2 : e3))));
-	if (!dev_out && d_perm) {TW_CUDA(ctx, cudaMemcpy(out, d_out, n*sizeof(float), cudaMemcpyDeviceToHost));} // schedule order scatters a chunk over the whole buffer: one copy at the end
+	if (host_out && d_perm) {TW_CUDA(ctx, cudaMemcpy(out, d_out, n*sizeof(float), cudaMemcpyDeviceToHost));} // schedule order scatters a chunk over the whole buffer: one copy at the end
 	unsigned long long h_steps = 0;
 	TW_CUDA(ctx, cudaMemcpy(&h_steps, d_steps, sizeof(h_steps), cudaMemcpyDeviceToHost));
 	ctx->last_erosion_steps = h_steps;
@@ -538,52 +541,42 @@ int tw_create_zvals_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t ntile
 }
 
 int tw_heightmap_sample_tiles(tw_ctx *ctx, const uint8_t *data16, const tw_hmap_sampler *hs, const int32_t *origins_xy, uint32_t ntiles, uint32_t zvsize, float *out) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!data16 || !hs || !origins_xy || !out || ntiles == 0 || zvsize == 0) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	if (hs->width <= 0 || hs->height <= 0 || hs->edge_mode < 0 || hs->edge_mode > 2) return tw_set_error(ctx, TW_ERR_ARG, "bad heightmap sampler");
 	if (ntiles > 65535) return tw_set_error(ctx, TW_ERR_ARG, "at most 65535 tiles per call");
-	size_t const img_bytes = ((size_t)2*hs->width*hs->height + 255) & ~(size_t)255, org_bytes = ((size_t)ntiles*8 + 255) & ~(size_t)255;
-	size_t const out_bytes = (size_t)ntiles*zvsize*zvsize*sizeof(float);
-	bool const dev_img = tw_is_device_ptr(data16), dev_out = tw_is_device_ptr(out);
-	rc = tw_reserve(ctx, 0, org_bytes + (dev_img ? 0 : img_bytes) + (dev_out ? 0 : out_bytes) + 256); if (rc) return rc;
-	char *sp = (char *)ctx->d_scratch[0];
-	void *d_org = sp; sp += org_bytes;
+	int32_t *d_org; const uint8_t *d_img; float *d_out;
+	tw_stage st(ctx);
+	st.temp(&d_org, (size_t)ntiles*8); // origins_xy is a host array
+	st.in(&d_img, data16, (size_t)2*hs->width*hs->height);
+	st.out(&d_out, out, (size_t)ntiles*zvsize*zvsize*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
 	TW_CUDA(ctx, cudaMemcpyAsync(d_org, origins_xy, (size_t)ntiles*8, cudaMemcpyHostToDevice, ctx->stream));
-	const uint8_t *d_img = data16;
-	if (!dev_img) {TW_CUDA(ctx, cudaMemcpyAsync(sp, data16, (size_t)2*hs->width*hs->height, cudaMemcpyHostToDevice, ctx->stream)); d_img = (const uint8_t *)sp; sp += img_bytes;}
-	float *d_out = dev_out ? out : (float *)sp;
 	rc = twi_hmap_sample_tiles(ctx, d_img, hs, d_org, ntiles, zvsize, d_out); if (rc) return rc;
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // origins_xy is the caller's buffer
-	return TW_OK;
+	return st.finish(); // also waits for the read of origins_xy, the caller's buffer
 }
 
 // ------------------------------------------------------------------------------------------------ per-tile normals and ambient occlusion (N1)
 int tw_tile_normals_batch(tw_ctx *ctx, const float *zvals, uint32_t ntiles, uint32_t zvsize, float dx_val, float dy_val, uint8_t *rgba, float *min_normal_z) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!zvals || !rgba || ntiles == 0 || zvsize < 2) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	if (ntiles > 65535) return tw_set_error(ctx, TW_ERR_ARG, "at most 65535 tiles per call");
-	size_t const n = (size_t)ntiles*zvsize*zvsize, stride = zvsize - 1, out_bytes = (size_t)ntiles*stride*stride*4;
-	bool const dev_in = tw_is_device_ptr(zvals), dev_out = tw_is_device_ptr(rgba);
-	size_t const in_bytes = (n*sizeof(float) + 255) & ~(size_t)255, mn_bytes = ((size_t)ntiles*sizeof(unsigned) + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, (dev_in ? 0 : in_bytes) + (dev_out ? 0 : out_bytes) + mn_bytes + 256); if (rc) return rc;
-	char *sp = (char *)ctx->d_scratch[0];
-	unsigned *d_mn = (unsigned *)sp; sp += mn_bytes;
-	const float *d_z = zvals;
-	if (!dev_in) {TW_CUDA(ctx, cudaMemcpyAsync(sp, zvals, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_z = (const float *)sp; sp += in_bytes;}
-	unsigned char *d_rgba = dev_out ? rgba : (unsigned char *)sp;
+	size_t const stride = zvsize - 1;
+	unsigned *d_mn; const float *d_z; uint8_t *d_rgba;
+	tw_stage st(ctx);
+	st.temp(&d_mn, (size_t)ntiles*sizeof(unsigned));
+	st.in(&d_z, zvals, (size_t)ntiles*zvsize*zvsize*sizeof(float));
+	st.out(&d_rgba, rgba, (size_t)ntiles*stride*stride*4);
+	rc = st.commit(); if (rc) return rc;
 	{
 		std::vector<unsigned> init(ntiles, tw_f2ord(1.0f)); // min_normal_z = 1.0, src/tiled_mesh.cpp:868
 		TW_CUDA(ctx, cudaMemcpyAsync(d_mn, init.data(), ntiles*sizeof(unsigned), cudaMemcpyHostToDevice, ctx->stream));
 		TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
 	}
 	rc = twi_tile_normals(ctx, d_z, ntiles, zvsize, dx_val, dy_val, d_rgba, d_mn); if (rc) return rc;
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(rgba, d_rgba, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));}
 	std::vector<unsigned> mn(ntiles);
 	if (min_normal_z) {TW_CUDA(ctx, cudaMemcpyAsync(mn.data(), d_mn, ntiles*sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	rc = st.finish(); if (rc) return rc;
 	if (min_normal_z) {for (uint32_t t = 0; t < ntiles; ++t) {min_normal_z[t] = tw_ord2f(mn[t]);}}
 	return TW_OK;
 }
@@ -595,7 +588,7 @@ static int gen_ao_contexts(tw_ctx *ctx, const int32_t *origins_xy, uint32_t nt, 
 	uint32_t const ray = 36, csz = zvsize - 1 + 2*ray; // AO_RAY_LEN, context_sz (src/tiled_mesh.cpp:43,601)
 	for (uint32_t t = 0; t < nt; ++t) {org[2*t] = origins_xy[2*t] - (int32_t)ray; org[2*t + 1] = origins_xy[2*t + 1] - (int32_t)ray;}
 	if (skip_inside) {ctx->skip_rect[0] = ctx->skip_rect[1] = ray; ctx->skip_rect[2] = ctx->skip_rect[3] = zvsize;}
-	int const rc = tw_heightgen_tiles(ctx, org.data(), nt, mesh_x_size, mesh_y_size, dx, dy, csz, p, d_cz, nullptr); // device output: scratch slot 0 is not touched
+	int const rc = tw_heightgen_tiles(ctx, org.data(), nt, mesh_x_size, mesh_y_size, dx, dy, csz, p, d_cz, nullptr); // device output: stages nothing in the caller's slot 0
 	ctx->skip_rect[0] = ctx->skip_rect[1] = ctx->skip_rect[2] = ctx->skip_rect[3] = 0;
 	return rc;
 }
@@ -603,31 +596,30 @@ static int gen_ao_contexts(tw_ctx *ctx, const int32_t *origins_xy, uint32_t nt, 
 int tw_tile_ao_batch(tw_ctx *ctx, const float *zvals, const int32_t *origins_xy, uint32_t ntiles, int mesh_x_size, int mesh_y_size,
                      float dx, float dy, uint32_t zvsize, const tw_height_params *p, float half_dxy, uint8_t *ao)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!zvals || !origins_xy || !p || !ao || ntiles == 0 || zvsize < 2) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	uint32_t const ray = 36, stride = zvsize - 1, csz = stride + 2*ray; // AO_RAY_LEN, context_sz (src/tiled_mesh.cpp:43,601)
 	size_t const tile_elems = (size_t)zvsize*zvsize, ctx_elems = (size_t)csz*csz, ao_elems = (size_t)stride*stride;
-	bool const dev_in = tw_is_device_ptr(zvals), dev_out = tw_is_device_ptr(ao);
 	bool const ctx_inside = (p->gen_mode >= TW_MGEN_SIMPLEX_GPU); // use_ao_zvals: the rays test the un-eroded context inside the tile too (src/tiled_mesh.cpp:604)
 	// chunk of tiles whose context grids fit in ~2 GB
 	uint32_t chunk = (uint32_t)std::min<size_t>(ntiles, std::max<size_t>(1, ((size_t)2 << 30)/(ctx_elems*sizeof(float))));
 	if (chunk > 65535) chunk = 65535;
-	size_t const in_bytes = ((size_t)chunk*tile_elems*sizeof(float) + 255) & ~(size_t)255, cz_bytes = ((size_t)chunk*ctx_elems*sizeof(float) + 255) & ~(size_t)255;
-	size_t const ao_bytes = ((size_t)chunk*ao_elems + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, (dev_in ? 0 : in_bytes) + cz_bytes + (dev_out ? 0 : ao_bytes) + 256); if (rc) return rc;
+	const float *z_buf; uint8_t *ao_buf; float *d_cz; // host zvals / ao: one chunk's region, device ones: the whole buffer
+	tw_stage st(ctx);
+	bool const host_z = st.view(&z_buf, zvals, (size_t)chunk*tile_elems*sizeof(float));
+	st.temp(&d_cz, (size_t)chunk*ctx_elems*sizeof(float));
+	bool const host_ao = st.view(&ao_buf, ao, (size_t)chunk*ao_elems);
+	rc = st.commit(); if (rc) return rc;
 	std::vector<int32_t> org(2*(size_t)chunk);
 	for (uint32_t t0 = 0; t0 < ntiles; t0 += chunk) {
 		uint32_t const nt = (ntiles - t0 < chunk) ? ntiles - t0 : chunk;
-		char *sp = (char *)ctx->d_scratch[0];
-		float *d_cz = (float *)sp; sp += cz_bytes;
-		const float *d_z = zvals + (size_t)t0*tile_elems;
-		if (!dev_in) {TW_CUDA(ctx, cudaMemcpyAsync(sp, d_z, (size_t)nt*tile_elems*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_z = (const float *)sp; sp += in_bytes;}
-		unsigned char *d_ao = dev_out ? ao + (size_t)t0*ao_elems : (unsigned char *)sp;
+		const float *d_z = host_z ? z_buf : zvals + (size_t)t0*tile_elems;
+		uint8_t *d_ao = host_ao ? ao_buf : ao + (size_t)t0*ao_elems;
+		if (host_z) {TW_CUDA(ctx, cudaMemcpyAsync(const_cast<float *>(z_buf), zvals + (size_t)t0*tile_elems, (size_t)nt*tile_elems*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));}
 		rc = gen_ao_contexts(ctx, origins_xy + 2*(size_t)t0, nt, mesh_x_size, mesh_y_size, dx, dy, zvsize, p, !ctx_inside, org, d_cz);
 		if (rc) return rc;
 		rc = twi_tile_ao(ctx, d_z, d_cz, nt, zvsize, half_dxy, ctx_inside, d_ao); if (rc) return rc;
-		if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(ao + (size_t)t0*ao_elems, d_ao, (size_t)nt*ao_elems, cudaMemcpyDeviceToHost, ctx->stream));}
+		if (host_ao) {TW_CUDA(ctx, cudaMemcpyAsync(ao + (size_t)t0*ao_elems, d_ao, (size_t)nt*ao_elems, cudaMemcpyDeviceToHost, ctx->stream));}
 		TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
 	}
 	return TW_OK;
@@ -637,30 +629,28 @@ int tw_create_zvals_ao_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t nt
                              uint32_t zvsize, const tw_height_params *p, uint32_t erosion_iters, const tw_erosion_params *ep, float min_zval,
                              float half_dxy, float *zvals, uint8_t *ao, tw_minmax *mm)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!origins_xy || !p || !zvals || !ao || ntiles == 0 || zvsize < 2) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	uint32_t const ray = 36, stride = zvsize - 1, csz = stride + 2*ray;
 	size_t const tile_elems = (size_t)zvsize*zvsize, ctx_elems = (size_t)csz*csz, ao_elems = (size_t)stride*stride;
-	bool const dev_z = tw_is_device_ptr(zvals), dev_ao = tw_is_device_ptr(ao);
 	bool const ctx_mode = (p->gen_mode >= TW_MGEN_SIMPLEX_GPU); // one generation, zvals cut from the context (src/tiled_mesh.cpp:479-487,505)
 	bool const erode = (erosion_iters > 0 && ep && ep->erode_amount > 0.0);
 	uint32_t chunk = (uint32_t)std::min<size_t>(ntiles, std::max<size_t>(1, ((size_t)2 << 30)/(ctx_elems*sizeof(float))));
 	if (chunk > 65535) chunk = 65535;
-	size_t const z_bytes = ((size_t)chunk*tile_elems*sizeof(float) + 255) & ~(size_t)255, cz_bytes = ((size_t)chunk*ctx_elems*sizeof(float) + 255) & ~(size_t)255;
-	size_t const ao_bytes = ((size_t)chunk*ao_elems + 255) & ~(size_t)255, mm_bytes = ((size_t)chunk*2*sizeof(unsigned) + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, cz_bytes + mm_bytes + (dev_z ? 0 : z_bytes) + (dev_ao ? 0 : ao_bytes) + 256); if (rc) return rc;
+	float *d_cz, *z_buf; unsigned *d_mm; uint8_t *ao_buf; // host zvals / ao: one chunk's region, device ones: the whole buffer
+	tw_stage st(ctx);
+	st.temp(&d_cz, (size_t)chunk*ctx_elems*sizeof(float));
+	st.temp(&d_mm, (size_t)chunk*2*sizeof(unsigned));
+	bool const host_z = st.view(&z_buf, zvals, (size_t)chunk*tile_elems*sizeof(float));
+	bool const host_ao = st.view(&ao_buf, ao, (size_t)chunk*ao_elems);
+	rc = st.commit(); if (rc) return rc;
 	std::vector<int32_t> org(2*(size_t)chunk);
 	uint64_t moves = 0;
 	for (uint32_t t0 = 0; t0 < ntiles; t0 += chunk) {
 		uint32_t const nt = (ntiles - t0 < chunk) ? ntiles - t0 : chunk;
 		const int32_t *orgs = origins_xy + 2*(size_t)t0;
-		char *sp = (char *)ctx->d_scratch[0];
-		float *d_cz = (float *)sp; sp += cz_bytes;
-		unsigned *d_mm = (unsigned *)sp; sp += mm_bytes;
-		float *d_z = dev_z ? zvals + (size_t)t0*tile_elems : (float *)sp;
-		if (!dev_z) {sp += z_bytes;}
-		unsigned char *d_ao = dev_ao ? ao + (size_t)t0*ao_elems : (unsigned char *)sp;
+		float *d_z = host_z ? z_buf : zvals + (size_t)t0*tile_elems;
+		uint8_t *d_ao = host_ao ? ao_buf : ao + (size_t)t0*ao_elems;
 		if (ctx_mode) {
 			rc = gen_ao_contexts(ctx, orgs, nt, mesh_x_size, mesh_y_size, dx, dy, zvsize, p, false, org, d_cz); if (rc) return rc;
 			rc = twi_tile_cut(ctx, d_cz, nt, zvsize, d_z); if (rc) return rc;
@@ -676,8 +666,8 @@ int tw_create_zvals_ao_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t nt
 			rc = twi_init_minmax(ctx, d_mm, nt); if (rc) return rc;
 			rc = twi_minmax_tiles(ctx, ctx->stream, d_z, tile_elems, nt, d_mm); if (rc) return rc;
 		}
-		if (!dev_z)  {TW_CUDA(ctx, cudaMemcpyAsync(zvals + (size_t)t0*tile_elems, d_z, (size_t)nt*tile_elems*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
-		if (!dev_ao) {TW_CUDA(ctx, cudaMemcpyAsync(ao + (size_t)t0*ao_elems, d_ao, (size_t)nt*ao_elems, cudaMemcpyDeviceToHost, ctx->stream));}
+		if (host_z)  {TW_CUDA(ctx, cudaMemcpyAsync(zvals + (size_t)t0*tile_elems, d_z, (size_t)nt*tile_elems*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
+		if (host_ao) {TW_CUDA(ctx, cudaMemcpyAsync(ao + (size_t)t0*ao_elems, d_ao, (size_t)nt*ao_elems, cudaMemcpyDeviceToHost, ctx->stream));}
 		if (mm) {rc = read_minmax(ctx, d_mm, mm + t0, nt); if (rc) return rc;}
 		TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
 	}
@@ -687,27 +677,17 @@ int tw_create_zvals_ao_batch(tw_ctx *ctx, const int32_t *origins_xy, uint32_t nt
 
 // ------------------------------------------------------------------------------------------------ point queries
 int tw_eval_points(tw_ctx *ctx, const float *xy, size_t n, const tw_height_params *p, const tw_point_query *q, float *out) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!xy || !p || !q || !out) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
 	if (n == 0) return TW_OK;
 	if (!ctx->have_sin) return tw_set_error(ctx, TW_ERR_STATE, "tw_set_sin_table() has not been called");
-	bool const dev_in = tw_is_device_ptr(xy), dev_out = tw_is_device_ptr(out);
-	size_t const in_bytes = (2*n*sizeof(float) + 255) & ~(size_t)255, out_bytes = n*sizeof(float);
-	size_t const need = (dev_in ? 0 : in_bytes) + (dev_out ? 0 : out_bytes);
-	if (need) {rc = tw_reserve(ctx, 0, need); if (rc) return rc;}
-	const float *d_xy = xy; float *d_out = out;
-	char *sp = (char *)ctx->d_scratch[0];
-	if (!dev_in) {
-		d_xy = (const float *)sp; sp += in_bytes;
-		TW_CUDA(ctx, cudaMemcpyAsync((void *)d_xy, xy, 2*n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-	}
-	if (!dev_out) {d_out = (float *)sp;}
-	rc = twi_eval_points(ctx, d_xy, n, p, q, d_out);
-	if (rc) return rc;
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	const float *d_xy; float *d_out;
+	tw_stage st(ctx);
+	st.in(&d_xy, xy, 2*n*sizeof(float));
+	st.out(&d_out, out, n*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	rc = twi_eval_points(ctx, d_xy, n, p, q, d_out); if (rc) return rc;
+	return st.finish();
 }
 
 int tw_erode(tw_ctx *ctx, float *heightmap, int xsize, int ysize, float min_zval, uint32_t num_iters, const tw_erosion_params *p) {
@@ -715,110 +695,81 @@ int tw_erode(tw_ctx *ctx, float *heightmap, int xsize, int ysize, float min_zval
 }
 
 int tw_erode_parallel(tw_ctx *ctx, float *heightmap, int xsize, int ysize, float min_zval, uint32_t num_iters, const tw_erosion_params *p, uint32_t num_threads) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!heightmap || !p) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
 	if (xsize <= 0 || ysize <= 0) return tw_set_error(ctx, TW_ERR_ARG, "empty heightmap");
 	if (num_iters == 0 || p->erode_amount <= 0.0) {ctx->last_erosion_steps = 0; return TW_OK;} // src/erosion.cpp:16
-	size_t const n = (size_t)xsize*ysize;
-	bool const dev = tw_is_device_ptr(heightmap);
-	float *d_map = heightmap;
-	if (!dev) {
-		rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc;
-		d_map = (float *)ctx->d_scratch[0];
-		TW_CUDA(ctx, cudaMemcpyAsync(d_map, heightmap, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-	}
-	rc = twi_erode_parallel(ctx, d_map, xsize, ysize, min_zval, num_iters, p, num_threads);
-	if (rc) return rc;
-	if (!dev) {TW_CUDA(ctx, cudaMemcpyAsync(heightmap, d_map, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	float *d_map;
+	tw_stage st(ctx);
+	st.inout(&d_map, heightmap, (size_t)xsize*ysize*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	rc = twi_erode_parallel(ctx, d_map, xsize, ysize, min_zval, num_iters, p, num_threads); if (rc) return rc;
+	return st.finish();
 }
 
 // ------------------------------------------------------------------------------------------------ voxels
 int tw_voxel_fill(tw_ctx *ctx, const tw_voxel_params *vp, const float *rdata420, float *out) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!vp || !out) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
 	if (!ctx->have_sin) return tw_set_error(ctx, TW_ERR_STATE, "tw_set_sin_table() has not been called");
 	if (vp->gen_mode < 0 || vp->gen_mode > TW_MGEN_DWARP_GPU) return tw_set_error(ctx, TW_ERR_ARG, "bad gen_mode");
-	size_t const n = (size_t)vp->nx*vp->ny*vp->nz;
-	bool const dev_out = tw_is_device_ptr(out);
-	float *d_out = out;
-	if (!dev_out) {rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc; d_out = (float *)ctx->d_scratch[0];}
-	rc = twi_voxel_fill(ctx, vp, rdata420, d_out);
-	if (rc) return rc;
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(out, d_out, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	float *d_out;
+	tw_stage st(ctx);
+	st.out(&d_out, out, (size_t)vp->nx*vp->ny*vp->nz*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	rc = twi_voxel_fill(ctx, vp, rdata420, d_out); if (rc) return rc;
+	return st.finish();
 }
 
 // ------------------------------------------------------------------------------------------------ streaming passes
 int tw_heightmap_from_floats_u16(tw_ctx *ctx, const float *vals, size_t n, float val_mult, float val_add, uint8_t *out2n) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!vals || !out2n || n == 0) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
-	bool const dev_in = tw_is_device_ptr(vals), dev_out = tw_is_device_ptr(out2n);
-	size_t const in_bytes = n*sizeof(float), out_bytes = 2*n;
-	size_t const need = (dev_in ? 0 : in_bytes) + (dev_out ? 0 : out_bytes);
-	if (need) {rc = tw_reserve(ctx, 0, need + 256); if (rc) return rc;}
+	const float *d_in; uint8_t *d_out;
+	tw_stage st(ctx);
+	st.in(&d_in, vals, n*sizeof(float));
+	st.out(&d_out, out2n, 2*n);
+	rc = st.commit(); if (rc) return rc;
 	rc = tw_reserve(ctx, 2, OFF_TILES); if (rc) return rc;
-	const float *d_in = vals; uint8_t *d_out = out2n;
-	char *s = (char *)ctx->d_scratch[0];
-	if (!dev_in) {d_in = (const float *)s; TW_CUDA(ctx, cudaMemcpyAsync(s, vals, in_bytes, cudaMemcpyHostToDevice, ctx->stream)); s += (in_bytes + 255) & ~(size_t)255;}
-	if (!dev_out) {d_out = (uint8_t *)s;}
 	unsigned *d_bad = (unsigned *)((char *)ctx->d_scratch[2] + OFF_BAD);
 	TW_CUDA(ctx, cudaMemsetAsync(d_bad, 0, sizeof(unsigned), ctx->stream));
 	rc = twi_from_floats_u16(ctx, d_in, n, val_mult, val_add, d_out, d_bad);
 	if (rc) return rc;
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(out2n, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));}
 	unsigned bad = 0;
 	TW_CUDA(ctx, cudaMemcpyAsync(&bad, d_bad, sizeof(bad), cudaMemcpyDeviceToHost, ctx->stream));
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	rc = st.finish(); if (rc) return rc;
 	if (bad) return tw_set_error(ctx, TW_ERR_ARG, "from_floats: value outside [0,256) (the reference asserts, src/heightmap.cpp:211)");
 	return TW_OK;
 }
 
 int tw_heightmap_to_floats_u16(tw_ctx *ctx, const uint8_t *data2n, size_t n, float val_mult, float val_add, float *vals) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!vals || !data2n || n == 0) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
-	bool const dev_in = tw_is_device_ptr(data2n), dev_out = tw_is_device_ptr(vals);
-	size_t const in_bytes = 2*n, out_bytes = n*sizeof(float);
-	size_t const need = (dev_in ? 0 : in_bytes) + (dev_out ? 0 : out_bytes);
-	if (need) {rc = tw_reserve(ctx, 0, need + 256); if (rc) return rc;}
-	const uint8_t *d_in = data2n; float *d_out = vals;
-	char *s = (char *)ctx->d_scratch[0];
-	if (!dev_out) {d_out = (float *)s; s += (out_bytes + 255) & ~(size_t)255;}
-	if (!dev_in) {d_in = (const uint8_t *)s; TW_CUDA(ctx, cudaMemcpyAsync(s, data2n, in_bytes, cudaMemcpyHostToDevice, ctx->stream));}
-	rc = twi_to_floats_u16(ctx, d_in, n, val_mult, val_add, d_out);
-	if (rc) return rc;
-	if (!dev_out) {TW_CUDA(ctx, cudaMemcpyAsync(vals, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	const uint8_t *d_in; float *d_out;
+	tw_stage st(ctx);
+	st.in(&d_in, data2n, 2*n);
+	st.out(&d_out, vals, n*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	rc = twi_to_floats_u16(ctx, d_in, n, val_mult, val_add, d_out); if (rc) return rc;
+	return st.finish();
 }
 
 int tw_proc_gen_heightmap(tw_ctx *ctx, uint32_t width, uint32_t height, float dx_val, float dy_val, const tw_height_params *p,
                           uint32_t erosion_iters, const tw_erosion_params *ep, uint8_t *data16, float *vals, tw_heightmap_info *info)
 {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!p || !data16 || width == 0 || height == 0) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
 	tw_grid2d g; g.x0 = -0.5*width; g.y0 = -0.5*height; g.dx = dx_val; g.dy = dy_val; g.nx = width; g.ny = height; // src/heightmap.cpp:135
 	size_t const n = (size_t)width*height;
-	bool const vals_dev = (vals && tw_is_device_ptr(vals)), out_dev = tw_is_device_ptr(data16);
-	// slot 0: [vals (if not given on the device)] [u16 image (if not given on the device)]
-	size_t const vbytes = (n*sizeof(float) + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, (vals_dev ? 0 : vbytes) + (out_dev ? 0 : 2*n) + 256); if (rc) return rc;
-	char *s0 = (char *)ctx->d_scratch[0];
-	float *d_vals = vals_dev ? vals : (float *)s0;
-	if (!vals_dev) {s0 += vbytes;}
-	uint8_t *d_img = out_dev ? data16 : (uint8_t *)s0;
+	float *d_vals; uint8_t *d_img;
+	tw_stage st(ctx);
+	if (vals) {st.out(&d_vals, vals, n*sizeof(float));} else {st.temp(&d_vals, n*sizeof(float));}
+	st.out(&d_img, data16, 2*n);
+	rc = st.commit(); if (rc) return rc;
 	rc = validate_height(ctx, &g, p, d_vals); if (rc) return rc;
-	rc = tw_reserve(ctx, 2, OFF_TILES); if (rc) return rc;
-	unsigned *d_mm = (unsigned *)((char *)ctx->d_scratch[2] + OFF_MM);
+	unsigned *d_mm;
 	tw_minmax mm;
-	rc = twi_init_minmax(ctx, d_mm, 1); if (rc) return rc;
+	rc = single_minmax(ctx, &d_mm); if (rc) return rc;
 	rc = twi_heightgen(ctx, &g, p, 1, 0, nullptr, 1, d_vals, d_mm); if (rc) return rc;
 	rc = read_minmax(ctx, d_mm, &mm, 1); if (rc) return rc;
 	uint64_t moves = 0;
@@ -840,11 +791,9 @@ int tw_proc_gen_heightmap(tw_ctx *ctx, uint32_t width, uint32_t height, float dx
 	unsigned *d_bad = (unsigned *)((char *)ctx->d_scratch[2] + OFF_BAD);
 	TW_CUDA(ctx, cudaMemsetAsync(d_bad, 0, sizeof(unsigned), ctx->stream));
 	rc = twi_from_floats_u16(ctx, d_vals, n, val_mult, val_add, d_img, d_bad); if (rc) return rc;
-	if (!out_dev) {TW_CUDA(ctx, cudaMemcpyAsync(data16, d_img, 2*n, cudaMemcpyDeviceToHost, ctx->stream));}
-	if (vals && !vals_dev) {TW_CUDA(ctx, cudaMemcpyAsync(vals, d_vals, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
 	unsigned bad = 0;
 	TW_CUDA(ctx, cudaMemcpyAsync(&bad, d_bad, sizeof(bad), cudaMemcpyDeviceToHost, ctx->stream));
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	rc = st.finish(); if (rc) return rc;
 	ctx->last_erosion_steps = moves;
 	if (info) {info->min_z = min_z; info->max_z = max_z; info->val_mult = val_mult; info->val_add = val_add; info->mesh_file_scale = mesh_file_scale; info->mesh_file_tz = mesh_file_tz; info->erosion_moves = moves;}
 	if (bad) return tw_set_error(ctx, TW_ERR_ARG, "from_floats: value outside [0,256) (the reference asserts, src/heightmap.cpp:211)");
@@ -852,18 +801,14 @@ int tw_proc_gen_heightmap(tw_ctx *ctx, uint32_t width, uint32_t height, float dx
 }
 
 int tw_minmax_f32(tw_ctx *ctx, const float *vals, size_t n, tw_minmax *mm) {
-	int rc = check_ctx(ctx); if (rc) return rc;
-	rc = finish_pending(ctx); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
 	if (!vals || !mm || n == 0) return tw_set_error(ctx, TW_ERR_ARG, "null/empty argument");
-	const float *d_in = vals;
-	if (!tw_is_device_ptr(vals)) {
-		rc = tw_reserve(ctx, 0, n*sizeof(float)); if (rc) return rc;
-		TW_CUDA(ctx, cudaMemcpyAsync(ctx->d_scratch[0], vals, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-		d_in = (const float *)ctx->d_scratch[0];
-	}
-	rc = tw_reserve(ctx, 2, OFF_TILES); if (rc) return rc;
-	unsigned *d_mm = (unsigned *)((char *)ctx->d_scratch[2] + OFF_MM);
-	rc = twi_init_minmax(ctx, d_mm, 1); if (rc) return rc;
+	const float *d_in;
+	tw_stage st(ctx);
+	st.in(&d_in, vals, n*sizeof(float));
+	rc = st.commit(); if (rc) return rc;
+	unsigned *d_mm;
+	rc = single_minmax(ctx, &d_mm); if (rc) return rc;
 	rc = twi_minmax(ctx, d_in, n, d_mm); if (rc) return rc;
 	return read_minmax(ctx, d_mm, mm, 1);
 }

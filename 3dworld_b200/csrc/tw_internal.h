@@ -34,8 +34,9 @@ struct tw_ctx {
 	float   h_sine_params[TW_F_TABLE_SIZE*5];
 	bool have_sin = false, have_sine_params = false;
 	// growable device scratch
-	void  *d_scratch[3] = {nullptr, nullptr, nullptr}; // 0: generic output staging, 1: tables / padded heightmaps, 2: small (minmax, counters, origins)
+	void  *d_scratch[3] = {nullptr, nullptr, nullptr}; // 0: caller-buffer staging (tw_stage only), 1: tables / padded heightmaps, 2: small (minmax, counters, origins)
 	size_t scratch_bytes[3] = {0, 0, 0};
+	bool scratch0_held = false;  // a tw_stage of the running entry point has buffers in slot 0: an entry it calls must not stage into slot 0
 	// pinned host staging for small results
 	void  *h_pinned = nullptr;
 	size_t pinned_bytes = 0;
@@ -48,6 +49,37 @@ int  tw_set_error(tw_ctx *ctx, int status, const char *fmt, ...);
 int  tw_reserve(tw_ctx *ctx, int slot, size_t bytes);           // grow d_scratch[slot]; returns TW_OK / TW_ERR_CUDA
 int  tw_reserve_pinned(tw_ctx *ctx, size_t bytes);
 bool tw_is_device_ptr(const void *p);
+int  tw_enter(tw_ctx *ctx);  // first call of every entry point that works on ctx: selects ctx->device, completes a pending tw_heightgen_2d_launch
+
+inline size_t tw_align256(size_t b) {return (b + 255) & ~(size_t)255;}
+
+// Device views of one entry-point call's caller buffers, which include/tw3d.h lets be host or device memory. A device buffer (or null) is used in place;
+// a host buffer, and every temp(), gets its own 256-byte-aligned region of scratch slot 0. Declare the buffers, then commit() reserves slot 0 once,
+// assigns the device pointers and uploads in / inout; finish() downloads out / inout and synchronises ctx->stream. view() gives the region but leaves
+// the copies to the call site (chunked, banded or pipelined transfers). slack: bytes the region has beyond the copied size (word atomics on a flag tail).
+class tw_stage {
+public:
+	explicit tw_stage(tw_ctx *ctx) : ctx_(ctx) {}
+	~tw_stage() {if (held_) ctx_->scratch0_held = false;}
+	tw_stage(const tw_stage &) = delete;
+	tw_stage &operator=(const tw_stage &) = delete;
+	template<class T> void in   (const T **d, const T *caller, size_t bytes)        {add(d, caller, bytes, 0, IN);}
+	template<class T> void out  (T **d, T *caller, size_t bytes, size_t slack = 0)  {add(d, caller, bytes, slack, OUT);}
+	template<class T> void inout(T **d, T *caller, size_t bytes, size_t slack = 0)  {add(d, caller, bytes, slack, IN | OUT);}
+	template<class T> bool view (T **d, T *caller, size_t bytes)                    {return add(d, caller, bytes, 0, 0);} // true: caller is host memory
+	template<class T> void temp (T **d, size_t bytes)                               {add(d, nullptr, bytes, 0, TEMP);}
+	int commit();
+	int finish();
+	static bool is_host(const void *p) {return p && !tw_is_device_ptr(p);}
+private:
+	enum {IN = 1, OUT = 2, TEMP = 4, MAX_BUFFERS = 8};
+	struct entry {void *d; const void *caller; void *dev; size_t bytes, region; int dir; bool host;};
+	bool add(void *d, const void *caller, size_t bytes, size_t slack, int dir);
+	tw_ctx *ctx_;
+	entry e_[MAX_BUFFERS];
+	int n_ = 0;
+	bool held_ = false;
+};
 
 #define TW_CUDA(ctx, call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
 	return tw_set_error((ctx), TW_ERR_CUDA, "%s:%d %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); } } while (0)

@@ -119,12 +119,11 @@ __global__ void shadow_unpack_kernel(const unsigned long long *__restrict__ kx, 
 extern "C" int tw_tile_shadows_batch(tw_ctx *ctx, const float *zvals, const int32_t *tile_xy, uint32_t ntiles, uint32_t zvsize, const tw_shadow_params *sp,
                                      uint8_t *smask, float *sh_out_x, float *sh_out_y)
 {
-	if (!ctx || !zvals || !tile_xy || !sp || !smask || ntiles == 0 || zvsize < 2) return TW_ERR_ARG;
-	TW_CUDA(ctx, cudaSetDevice(ctx->device));
+	int rc = tw_enter(ctx); if (rc) return rc;
+	if (!zvals || !tile_xy || !sp || !smask || ntiles == 0 || zvsize < 2) return tw_set_error(ctx, TW_ERR_ARG, "null argument, no tiles or zvsize < 2");
 	if (ntiles > 65535) return tw_set_error(ctx, TW_ERR_ARG, "at most 65535 tiles per call");
 	int const n = (int)zvsize;
 	size_t const cells = (size_t)ntiles*n*n, edge = (size_t)ntiles*n;
-	if ((cells & 3) && ntiles > 1) {/* tiles of odd cell count straddle flag words: still correct, the atomics are per word */}
 	// neighbours toward the light, dependency waves
 	int const sx = (sp->lpos[0] < 0.0f) ? -1 : 1, sy = (sp->lpos[1] < 0.0f) ? -1 : 1;
 	std::map<std::pair<int, int>, int> where;
@@ -166,26 +165,21 @@ extern "C" int tw_tile_shadows_batch(tw_ctx *ctx, const float *zvals, const int3
 		S.dim = (fabsf(S.dirx) < fabsf(S.diry)) ? 1 : 0;
 		S.dir_ratio = (double)(S.dirz/(S.dim ? S.diry : S.dirx));
 	}
-	bool const dev_z = tw_is_device_ptr(zvals), dev_m = tw_is_device_ptr(smask);
-	if (dev_m && ((size_t)smask & 3)) return tw_set_error(ctx, TW_ERR_ARG, "smask must be 4-byte aligned (flag bytes are set with 32-bit atomics)");
-	size_t const zb = (cells*sizeof(float) + 255) & ~(size_t)255, mb = (cells + 259) & ~(size_t)255, kb = (edge*sizeof(unsigned long long) + 255) & ~(size_t)255;
-	size_t const fb = (edge*sizeof(float) + 255) & ~(size_t)255, ib = ((size_t)ntiles*sizeof(int) + 255) & ~(size_t)255;
-	int rc = tw_reserve(ctx, 0, (dev_z ? 0 : zb) + (dev_m ? 0 : mb) + 2*kb + 2*fb + 3*ib + 256); if (rc) return rc;
-	char *p = (char *)ctx->d_scratch[0];
-	const float *d_z = zvals; unsigned char *d_m = smask;
-	if (!dev_z) {TW_CUDA(ctx, cudaMemcpyAsync(p, zvals, cells*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_z = (const float *)p; p += zb;}
-	if (!dev_m) {d_m = (unsigned char *)p; p += mb;}
-	unsigned long long *d_kx = (unsigned long long *)p; p += kb;
-	unsigned long long *d_ky = (unsigned long long *)p; p += kb;
-	float *d_ox = (float *)p; p += fb;
-	float *d_oy = (float *)p; p += fb;
-	int *d_wave = (int *)p; p += ib;
-	int *d_nbx = (int *)p; p += ib;
-	int *d_nby = (int *)p;
-	TW_CUDA(ctx, cudaMemcpyAsync(d_wave, wave_tiles.data(), (size_t)ntiles*sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-	TW_CUDA(ctx, cudaMemcpyAsync(d_nbx, nbx.data(), (size_t)ntiles*sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-	TW_CUDA(ctx, cudaMemcpyAsync(d_nby, nby.data(), (size_t)ntiles*sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-	shadow_init_kernel<<<148*8, 256, 0, ctx->stream>>>(d_m, d_kx, cells, 2*(kb/sizeof(unsigned long long)), all_shadowed ? (unsigned char)TW_MESH_SHADOW : (unsigned char)0);
+	size_t const nkeys = tw_align256(edge*sizeof(unsigned long long))/sizeof(unsigned long long); // keys of sh_out_x, then those of sh_out_y
+	const float *d_z; uint8_t *d_m; unsigned long long *d_kx; float *d_ox, *d_oy; const int *d_wave, *d_nbx, *d_nby;
+	tw_stage st(ctx);
+	st.in(&d_z, zvals, cells*sizeof(float));
+	st.out(&d_m, smask, cells, 4); // + 4: the rays set flag bytes with atomics on the 32-bit word that holds them
+	st.temp(&d_kx, 2*nkeys*sizeof(unsigned long long));
+	st.temp(&d_ox, edge*sizeof(float));
+	st.temp(&d_oy, edge*sizeof(float));
+	st.in(&d_wave, wave_tiles.data(), (size_t)ntiles*sizeof(int));
+	st.in(&d_nbx, nbx.data(), (size_t)ntiles*sizeof(int));
+	st.in(&d_nby, nby.data(), (size_t)ntiles*sizeof(int));
+	rc = st.commit(); if (rc) return rc;
+	if ((size_t)d_m & 3) return tw_set_error(ctx, TW_ERR_ARG, "smask must be 4-byte aligned (flag bytes are set with 32-bit atomics)"); // only a device buffer can be
+	unsigned long long *d_ky = d_kx + nkeys;
+	shadow_init_kernel<<<148*8, 256, 0, ctx->stream>>>(d_m, d_kx, cells, 2*nkeys, all_shadowed ? (unsigned char)TW_MESH_SHADOW : (unsigned char)0);
 	TW_LAUNCH_CHECK(ctx);
 	for (int l = 0; l < nlevels; ++l) {
 		int const nw = wave_start[l + 1] - wave_start[l];
@@ -196,9 +190,7 @@ extern "C" int tw_tile_shadows_batch(tw_ctx *ctx, const float *zvals, const int3
 		shadow_unpack_kernel<<<dim3((n + 127)/128, nw), 128, 0, ctx->stream>>>(d_kx, d_ky, d_ox, d_oy, n, d_wave + wave_start[l]);
 		TW_LAUNCH_CHECK(ctx);
 	}
-	if (!dev_m) {TW_CUDA(ctx, cudaMemcpyAsync(smask, d_m, cells, cudaMemcpyDeviceToHost, ctx->stream));}
 	if (sh_out_x) {TW_CUDA(ctx, cudaMemcpyAsync(sh_out_x, d_ox, edge*sizeof(float), cudaMemcpyDefault, ctx->stream));}
 	if (sh_out_y) {TW_CUDA(ctx, cudaMemcpyAsync(sh_out_y, d_oy, edge*sizeof(float), cudaMemcpyDefault, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	return st.finish();
 }

@@ -249,23 +249,19 @@ unsigned stream_grid(size_t n) {size_t const b = (n + 255)/256; return (unsigned
 } // namespace
 
 extern "C" int tw_voxel_outside(tw_ctx *ctx, const float *vals, const tw_voxel_post_params *vp, const uint32_t *zix_xy, uint8_t *outside) {
-	if (!ctx || !vals || !outside) return TW_ERR_ARG;
-	TW_CUDA(ctx, cudaSetDevice(ctx->device));
-	int rc = validate(ctx, vp); if (rc) return rc;
-	size_t const n = (size_t)vp->nx*vp->ny*vp->nz, nxy = (size_t)vp->nx*vp->ny;
-	bool const dev_v = tw_is_device_ptr(vals), dev_o = tw_is_device_ptr(outside), dev_z = (zix_xy && tw_is_device_ptr(zix_xy));
-	size_t const vb = (n*sizeof(float) + 255) & ~(size_t)255, ob = (n + 255) & ~(size_t)255, zb = (nxy*sizeof(unsigned) + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, (dev_v ? 0 : vb) + (dev_o ? 0 : ob) + ((zix_xy && !dev_z) ? zb : 0) + 256); if (rc) return rc;
-	char *sp = (char *)ctx->d_scratch[0];
-	const float *d_v = vals; uint8_t *d_o = outside; const unsigned *d_z = zix_xy;
-	if (!dev_v) {TW_CUDA(ctx, cudaMemcpyAsync(sp, vals, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_v = (const float *)sp; sp += vb;}
-	if (!dev_o) {d_o = (uint8_t *)sp; sp += ob;}
-	if (zix_xy && !dev_z) {TW_CUDA(ctx, cudaMemcpyAsync(sp, zix_xy, nxy*sizeof(unsigned), cudaMemcpyHostToDevice, ctx->stream)); d_z = (const unsigned *)sp;}
+	int rc = tw_enter(ctx); if (rc) return rc;
+	if (!vals || !outside) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
+	rc = validate(ctx, vp); if (rc) return rc;
+	size_t const n = (size_t)vp->nx*vp->ny*vp->nz;
+	const float *d_v; uint8_t *d_o; const uint32_t *d_z;
+	tw_stage st(ctx);
+	st.in(&d_v, vals, n*sizeof(float));
+	st.out(&d_o, outside, n);
+	st.in(&d_z, zix_xy, (size_t)vp->nx*vp->ny*sizeof(uint32_t));
+	rc = st.commit(); if (rc) return rc;
 	outside_kernel<<<stream_grid(n), 256, 0, ctx->stream>>>(d_v, *vp, d_z, d_o, n);
 	TW_LAUNCH_CHECK(ctx);
-	if (!dev_o) {TW_CUDA(ctx, cudaMemcpyAsync(outside, d_o, n, cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-	return TW_OK;
+	return st.finish();
 }
 
 // one flood fill: frontier buffers f[0], f[1] (n + 16 entries each), counters cnt[0], cnt[1]; the seeds are already in f[0] / cnt[0]
@@ -286,24 +282,23 @@ static int run_flood(tw_ctx *ctx, unsigned char *d_o, const tw_voxel_post_params
 }
 
 extern "C" int tw_voxel_remove_unconnected(tw_ctx *ctx, float *vals, uint8_t *outside, const tw_voxel_post_params *vp, uint64_t *changed) {
-	if (!ctx || !vals || !outside) return TW_ERR_ARG;
-	TW_CUDA(ctx, cudaSetDevice(ctx->device));
-	int rc = validate(ctx, vp); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
+	if (!vals || !outside) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
+	rc = validate(ctx, vp); if (rc) return rc;
 	if (changed) *changed = 0;
 	if (vp->remove_unconnected <= 0) return TW_OK;
 	size_t const n = (size_t)vp->nx*vp->ny*vp->nz;
-	bool const dev_v = tw_is_device_ptr(vals), dev_o = tw_is_device_ptr(outside);
-	if (dev_o && ((size_t)outside & 3)) return tw_set_error(ctx, TW_ERR_ARG, "outside must be 4-byte aligned (flag bytes are claimed with 32-bit atomics)");
-	size_t const vb = (n*sizeof(float) + 255) & ~(size_t)255, ob = (n + 255 + 4) & ~(size_t)255, fb = ((n + 16)*sizeof(unsigned) + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, (dev_v ? 0 : vb) + (dev_o ? 0 : ob) + 2*fb + 512); if (rc) return rc;
-	char *sp = (char *)ctx->d_scratch[0];
-	float *d_v = vals; unsigned char *d_o = outside;
-	if (!dev_v) {d_v = (float *)sp; sp += vb; TW_CUDA(ctx, cudaMemcpyAsync(d_v, vals, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream));}
-	if (!dev_o) {d_o = (unsigned char *)sp; sp += ob; TW_CUDA(ctx, cudaMemcpyAsync(d_o, outside, n, cudaMemcpyHostToDevice, ctx->stream));}
-	unsigned *f[2] = {(unsigned *)sp, (unsigned *)(sp + fb)}; sp += 2*fb;
-	unsigned *cnt = (unsigned *)sp;
-	unsigned long long *d_changed = (unsigned long long *)(sp + 64);
-	TW_CUDA(ctx, cudaMemsetAsync(sp, 0, 128, ctx->stream));
+	float *d_v; uint8_t *d_o; unsigned *f[2], *cnt;
+	tw_stage st(ctx);
+	st.inout(&d_v, vals, n*sizeof(float));
+	st.inout(&d_o, outside, n, 4); // + 4: claim() sets flag bytes with atomics on the 32-bit word that holds them
+	st.temp(&f[0], (n + 16)*sizeof(unsigned));
+	st.temp(&f[1], (n + 16)*sizeof(unsigned));
+	st.temp(&cnt, 128); // cnt[0], cnt[1]; the changed counter at byte 64
+	rc = st.commit(); if (rc) return rc;
+	if ((size_t)d_o & 3) return tw_set_error(ctx, TW_ERR_ARG, "outside must be 4-byte aligned (flag bytes are claimed with 32-bit atomics)"); // only a device buffer can be
+	unsigned long long *d_changed = (unsigned long long *)((char *)cnt + 64);
+	TW_CUDA(ctx, cudaMemsetAsync(cnt, 0, 128, ctx->stream));
 	// remove_unconnected_outside_range(keep_at_edge, 0, 0, nx, ny): anchors, fill of the inside voxels, verdict
 	if (vp->centre_seed) {seed_centre_kernel<<<1, 1, 0, ctx->stream>>>(d_o, *vp, f[0], cnt);}
 	else {seed_kernel<<<stream_grid(n), 256, 0, ctx->stream>>>(d_o, *vp, 0, f[0], cnt, n);}
@@ -327,9 +322,7 @@ extern "C" int tw_voxel_remove_unconnected(tw_ctx *ctx, float *vals, uint8_t *ou
 	}
 	unsigned long long hc = 0;
 	TW_CUDA(ctx, cudaMemcpyAsync(&hc, d_changed, sizeof(hc), cudaMemcpyDeviceToHost, ctx->stream));
-	if (!dev_v) {TW_CUDA(ctx, cudaMemcpyAsync(vals, d_v, n*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
-	if (!dev_o) {TW_CUDA(ctx, cudaMemcpyAsync(outside, d_o, n, cudaMemcpyDeviceToHost, ctx->stream));}
-	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+	rc = st.finish(); if (rc) return rc;
 	if (changed) *changed = hc;
 	return TW_OK;
 }
@@ -337,28 +330,22 @@ extern "C" int tw_voxel_remove_unconnected(tw_ctx *ctx, float *vals, uint8_t *ou
 extern "C" int tw_voxel_triangles(tw_ctx *ctx, const float *vals, const uint8_t *outside, const tw_voxel_post_params *vp, const uint32_t *edge_table256,
                                   const int32_t *tri_table256x16, const uint32_t *edge_to_vals12x2, float *tris, uint64_t capacity, uint64_t *ntris)
 {
-	if (!ctx || !vals || !outside || !edge_table256 || !tri_table256x16 || !edge_to_vals12x2 || !ntris || (capacity && !tris)) return TW_ERR_ARG;
-	TW_CUDA(ctx, cudaSetDevice(ctx->device));
-	int rc = validate(ctx, vp); if (rc) return rc;
+	int rc = tw_enter(ctx); if (rc) return rc;
+	if (!vals || !outside || !edge_table256 || !tri_table256x16 || !edge_to_vals12x2 || !ntris || (capacity && !tris)) return tw_set_error(ctx, TW_ERR_ARG, "null argument");
+	rc = validate(ctx, vp); if (rc) return rc;
 	size_t const n = (size_t)vp->nx*vp->ny*vp->nz;
 	unsigned const nblocks = (unsigned)((n + MC_BLOCK - 1)/MC_BLOCK);
-	bool const dev_v = tw_is_device_ptr(vals), dev_o = tw_is_device_ptr(outside), dev_t = (tris && tw_is_device_ptr(tris));
-	size_t const vb = (n*sizeof(float) + 255) & ~(size_t)255, ob = (n + 255) & ~(size_t)255, tb = 256*4 + 256*16*4 + 24*4 + 256;
-	size_t const sb = ((size_t)nblocks*sizeof(unsigned) + 255) & ~(size_t)255, ofb = ((size_t)nblocks*sizeof(unsigned long long) + 255) & ~(size_t)255;
-	rc = tw_reserve(ctx, 0, (dev_v ? 0 : vb) + (dev_o ? 0 : ob) + tb + sb + ofb + 512); if (rc) return rc;
-	char *sp = (char *)ctx->d_scratch[0];
-	const float *d_v = vals; const unsigned char *d_o = outside;
-	if (!dev_v) {TW_CUDA(ctx, cudaMemcpyAsync(sp, vals, n*sizeof(float), cudaMemcpyHostToDevice, ctx->stream)); d_v = (const float *)sp; sp += vb;}
-	if (!dev_o) {TW_CUDA(ctx, cudaMemcpyAsync(sp, outside, n, cudaMemcpyHostToDevice, ctx->stream)); d_o = (const unsigned char *)sp; sp += ob;}
-	McTables T;
-	T.edge_table = (const unsigned *)sp; T.tri_table = (const int *)(sp + 1024); T.edge_to_vals = (const unsigned *)(sp + 1024 + 16384);
-	TW_CUDA(ctx, cudaMemcpyAsync(sp, edge_table256, 1024, cudaMemcpyDefault, ctx->stream));
-	TW_CUDA(ctx, cudaMemcpyAsync(sp + 1024, tri_table256x16, 16384, cudaMemcpyDefault, ctx->stream));
-	TW_CUDA(ctx, cudaMemcpyAsync(sp + 1024 + 16384, edge_to_vals12x2, 96, cudaMemcpyDefault, ctx->stream));
-	sp += tb;
-	unsigned *d_sums = (unsigned *)sp; sp += sb;
-	unsigned long long *d_offsets = (unsigned long long *)sp; sp += ofb;
-	unsigned long long *d_total = (unsigned long long *)sp;
+	const float *d_v; const uint8_t *d_o; McTables T; unsigned *d_sums; unsigned long long *d_offsets, *d_total;
+	tw_stage st(ctx);
+	st.in(&d_v, vals, n*sizeof(float));
+	st.in(&d_o, outside, n);
+	st.in(&T.edge_table, edge_table256, 256*sizeof(uint32_t));
+	st.in(&T.tri_table, tri_table256x16, 256*16*sizeof(int32_t));
+	st.in(&T.edge_to_vals, edge_to_vals12x2, 12*2*sizeof(uint32_t));
+	st.temp(&d_sums, (size_t)nblocks*sizeof(unsigned));
+	st.temp(&d_offsets, (size_t)nblocks*sizeof(unsigned long long));
+	st.temp(&d_total, sizeof(unsigned long long));
+	rc = st.commit(); if (rc) return rc;
 	mc_kernel<false><<<nblocks, MC_BLOCK, 0, ctx->stream>>>(d_v, d_o, *vp, T, n, d_sums, nullptr, nullptr, 0);
 	TW_LAUNCH_CHECK(ctx);
 	scan_blocks_kernel<<<1, 1024, 0, ctx->stream>>>(d_sums, nblocks, d_offsets, d_total);
@@ -370,10 +357,11 @@ extern "C" int tw_voxel_triangles(tw_ctx *ctx, const float *vals, const uint8_t 
 	if (capacity == 0 || total == 0) return TW_OK;
 	uint64_t const nw = (total < capacity) ? total : capacity;
 	float *d_t = tris;
-	if (!dev_t) {rc = tw_reserve(ctx, 1, (size_t)nw*9*sizeof(float)); if (rc) return rc; d_t = (float *)ctx->d_scratch[1];}
+	bool const host_t = tw_stage::is_host(tris);
+	if (host_t) {rc = tw_reserve(ctx, 1, (size_t)nw*9*sizeof(float)); if (rc) return rc; d_t = (float *)ctx->d_scratch[1];}
 	mc_kernel<true><<<nblocks, MC_BLOCK, 0, ctx->stream>>>(d_v, d_o, *vp, T, n, nullptr, d_offsets, d_t, nw);
 	TW_LAUNCH_CHECK(ctx);
-	if (!dev_t) {TW_CUDA(ctx, cudaMemcpyAsync(tris, d_t, (size_t)nw*9*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
+	if (host_t) {TW_CUDA(ctx, cudaMemcpyAsync(tris, d_t, (size_t)nw*9*sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));}
 	TW_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
 	return TW_OK;
 }
